@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- per-round query throughput of the acquisition-scoring engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras] [--dump-outputs DIR]
 
 Headline (BASELINE.json configs[1]): MarginSampler query tail on an ImageNet-shaped pool of
 80 000 x 1000 fp32 logits per GPU, budget 10 000.  A "step" is one full tail: K1 (softmax margin)
@@ -19,6 +19,11 @@ roofline objects -- the BADGE k-means++ streaming kernel is the north star's 90 
 
 `--impl reference` times the reference's CPU implementation of the same tail (oracle port: the
 reference is Python and cannot travel to the GPU box) on all host threads.
+
+`--dump-outputs DIR` writes what the last timed step of the headline tail returned to its caller (rank 0's caller
+at N > 1): `scores.npy` (float32, this rank's 80 000 margins; not with --impl reference, whose tail returns only the
+positions) and `picks.npy` (the B selected positions, as float64).  The inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -221,8 +226,10 @@ def run_reference(args):
         cpu_margin_tail(logits, BUDGET)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_margin_tail(logits, BUDGET)
+        picks = cpu_margin_tail(logits, BUDGET)
     dt = (time.perf_counter() - t0) / max(args.steps, 1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, picks=picks)
     val = N_ROWS / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": "samples/s", "n_gpus": args.gpus,
@@ -237,6 +244,14 @@ def run_reference(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line))
+
+
+def dump_outputs(out_dir, **arrays):
+    """DIR/<name>.npy per array: floating arrays keep float32 / float64, integer ones (positions) become float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
 
 
 def host_cpu_budget():
@@ -813,6 +828,8 @@ def run_own(args):
     clocks.__enter__()
     clocks.wait_first(8.0 if rank == 0 else 0.0)
     R = run_region(1, args.steps, max(args.warmup, 3))
+    # the region ran on `scores`, so it holds the last timed step's margins until the next region overwrites it
+    dumped = {"scores": scores.cpu().numpy(), "picks": R["res"].numpy()} if args.dump_outputs else None
     t_w0, t_enq, t_w1 = R["t"]
     res, launches, ms_total, k1_ms = R["res"], R["launches"], R["ms_total"], R["k1_ms"]
     launches0 = eng.launches - launches
@@ -967,6 +984,8 @@ def run_own(args):
             torch.cuda.empty_cache()
         line["workloads"] = extras
         line["gpu_launches_total"] = int(eng.launches - launches0)
+    if dumped is not None and rank == 0:
+        dump_outputs(args.dump_outputs, **dumped)
     sys.stdout.flush()
     os.dup2(real_stdout, 1)
     if rank == 0:
@@ -985,7 +1004,10 @@ def main():
     ap.add_argument("--impl", default="own", choices=["own", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the CoreSet/BADGE workloads (N=1)")
     ap.add_argument("--extra-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

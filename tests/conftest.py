@@ -1,7 +1,6 @@
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,5 +30,5 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def gold():
-    path = os.path.join(ROOT, "tests", "golden", "reference_golden.npz")
-    return dict(np.load(path))
+    from helpers import load_gold
+    return load_gold()

@@ -120,6 +120,8 @@ def main():
         gold[f"margin_{tag}_logits"] = logits.numpy()
         gold[f"margin_{tag}_picks"] = np.array(idx, dtype=np.int64)
         assert cost == 60
+    # 2.8 MB: tests/helpers.py regenerates these logits from the seed and checks them against this sample
+    gold["margin_f32_c1000_logits_sample"] = gold.pop("margin_f32_c1000_logits")[::7, ::13]
 
     # ---------------------------------------------------------------- Confidence (A2)
     # As shipped the reference raises (confidence_sampler.py:41).  Record that, then record the

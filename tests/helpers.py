@@ -3,6 +3,7 @@ embeddings of every pool index, and OracleEngine -- an implementation of the Eng
 CPU tensors built from oracle/al_oracle.py.  OracleEngine exists ONLY so the CPU test tier can
 exercise the samplers' host logic (index bookkeeping, RNG order, partition batching, sharding);
 it is never importable from the product package."""
+import os
 import tempfile
 
 import numpy as np
@@ -10,6 +11,29 @@ import torch
 import torch.nn as nn
 
 from oracle import al_oracle as O
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_golden.npz")
+
+
+def c1000_logits():
+    """The 700 x 1000 logits of the f32_c1000 margin case (2.8 MB, too large to store).  make_golden.py drew them
+    from torch's CPU generator seeded with 0, after the f32_c10 logits and the one int64 seed that case's DataLoader
+    drew; this replays the same draws."""
+    g = torch.Generator().manual_seed(0)
+    torch.randn(700, 10, generator=g)
+    torch.empty((), dtype=torch.int64).random_(generator=g)
+    return torch.randn(700, 1000, generator=g) * 3.0
+
+
+def load_gold(path=GOLD):
+    """reference_golden.npz as a dict, with margin_f32_c1000_logits regenerated and checked against the strided
+    sample make_golden.py stored of it."""
+    gold = dict(np.load(path))
+    logits = c1000_logits().numpy()
+    assert np.array_equal(logits[::7, ::13], gold.pop("margin_f32_c1000_logits_sample")), \
+        "torch's CPU generator no longer reproduces the f32_c1000 logits"
+    gold["margin_f32_c1000_logits"] = logits
+    return gold
 
 
 class IndexDataset(torch.utils.data.Dataset):

@@ -1,42 +1,36 @@
 """INTEGRATION.md's three-line patch, executed: `make_drop_in` binds the accelerated query() implementations onto the
-REFERENCE's own `Strategy` (/root/reference/src/query_strategies/strategy.py:74), the resulting classes are built with
-the reference's constructor contract and their query() -- arithmetic by the CPU oracle engine, as everywhere in the
-CPU tier -- must return exactly what the reference's own samplers return on the same pool, labels and RNG seed.
-Runs where the reference checkout exists (the build container); skipped elsewhere."""
+Strategy base class it is given -- here the package's own query-path Strategy, which keeps the reference's
+constructor contract and bookkeeping -- and the resulting classes' query(), arithmetic by the CPU oracle engine as
+everywhere in the CPU tier, must return exactly what the reference's own samplers returned on the same pool, labels
+and RNG seed (recorded by tests/golden/make_golden_live.py in reference_golden_live.npz)."""
 import os
-import sys
 import tempfile
 
 import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference/src"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
-HERE = os.path.dirname(os.path.abspath(__file__))
+from active_learning_b200.integration import make_drop_in
+from active_learning_b200.query_strategies.strategy import Strategy
+
+LIVE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_golden_live.npz")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    sys.path.insert(0, os.path.join(HERE, "golden"))
-    import make_golden as G
-    get_strategy, Exp = G._import_reference()
-    import query_strategies.strategy as ref_strategy          # the reference's module, imported in place
-    from active_learning_b200.integration import make_drop_in
-    return dict(G=G, get_strategy=get_strategy, Exp=Exp, base=ref_strategy.Strategy, accel=make_drop_in(ref_strategy.Strategy))
+    return dict(np.load(LIVE))
 
 
-def _build(ref, cls, logits, emb, ev, lab, bs, **kw):
-    from helpers import OracleEngine
-    G = ref["G"]
+def _build(cls, exp, logits, emb, ev, lab, bs, **kw):
+    from helpers import IndexDataset, LookupNet, OracleEngine
     n, c = logits.shape
-    ds = G.IndexDataset(n, c)
-    net = G.LookupNet(logits, emb)
+    ds = IndexDataset(n, c)
+    net = LookupNet(logits, emb)
     args = dict(early_stop_patience=0, n_epoch=1, world_size=1, model="SSLResNet18", freeze_feature=True,
                 ckpt_path=tempfile.mkdtemp(prefix="dropin_"), exp_name="d", subset_labeled=None, subset_unlabeled=None,
                 partitions=1)
     args.update(kw)
-    s = cls(ds, ds, net, {"loader_te_args": {"batch_size": bs, "num_workers": 0}}, np.array(ev), ref["Exp"](), None, **args)
+    s = cls(ds, ds, net, {"loader_te_args": {"batch_size": bs, "num_workers": 0}}, np.array(ev), exp, None, **args)
     s.feature_net = s.net            # what the reference's init_network_weights does (strategy.py:198)
     if hasattr(s, "set_engine"):
         s.set_engine(OracleEngine())
@@ -55,8 +49,7 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("name,kw,budget", CASES)
-def test_drop_in_classes_on_the_reference_strategy_return_the_reference_picks(ref, name, kw, budget):
+def inputs():
     rng = np.random.default_rng(5)
     torch.manual_seed(5)
     n, c, d = 420, 10, 32
@@ -65,17 +58,22 @@ def test_drop_in_classes_on_the_reference_strategy_return_the_reference_picks(re
     lab = rng.choice(rest, size=70, replace=False)
     logits = torch.randn(n, c) * 3
     emb = torch.from_numpy(rng.integers(-2, 3, size=(n, d)).astype(np.float32))     # exact arithmetic: order-free sums
+    return logits, emb, ev, lab
 
-    mine = _build(ref, ref["accel"][name], logits, emb, ev, lab, 64, **kw)
-    theirs = _build(ref, ref["get_strategy"](name), logits, emb, ev, lab, 64, **kw)
-    # the accelerated class IS a reference Strategy: training, checkpointing, update() are the reference's own
-    assert isinstance(mine, ref["base"]) and ref["base"] in type(mine).__mro__
-    assert type(mine).train is ref["base"].train and type(mine).update is ref["base"].update
+
+@pytest.mark.parametrize("name,kw,budget", CASES)
+def test_drop_in_classes_on_the_reference_strategy_return_the_reference_picks(ref, name, kw, budget):
+    from helpers import FakeExperiment
+    case = CASES.index((name, kw, budget))
+    logits, emb, ev, lab = inputs()
+    accel = make_drop_in(Strategy)
+    mine = _build(accel[name], FakeExperiment(), logits, emb, ev, lab, 64, **kw)
+    # the accelerated class IS a Strategy of the base it was bound to: training, checkpointing, update() are the base's
+    assert isinstance(mine, Strategy) and Strategy in type(mine).__mro__
+    assert type(mine).train is Strategy.train and type(mine).update is Strategy.update
     np.random.seed(9)
     got, got_cost = mine.query(budget)
-    np.random.seed(9)
-    want, want_cost = theirs.query(budget)
-    assert [int(i) for i in got] == [int(i) for i in want] and got_cost == want_cost
-    # the consumer of query()'s return: the reference's update() accepts it (asserts not-yet-labeled, strategy.py:470)
+    assert [int(i) for i in got] == ref[f"dropin{case}_picks"].tolist() and got_cost == ref[f"dropin{case}_cost"]
+    # the consumer of query()'s return: update() accepts it (asserts not-yet-labeled, strategy.py:470)
     mine.update(got, got_cost)
     assert mine.idxs_lb[np.asarray(got, dtype=np.int64)].all()

@@ -1,6 +1,6 @@
 """Multi-GPU (one process per GPU, NCCL + peer-memory windows): results must equal the single-GPU /
-reference results for every world size.  Needs >= 2 GPUs (skipped otherwise; run with
-`gpurun --gpus 2 -- python -m pytest tests/test_gpu_multi.py -m gpu`)."""
+reference results for every world size.  Needs >= 2 GPUs (skipped otherwise; on a machine with two, run
+`python -m pytest tests/test_gpu_multi.py -m gpu`)."""
 import os
 import socket
 import sys
@@ -22,10 +22,10 @@ def _worker(rank, world, port, gold_path, out_path):
     os.environ["MASTER_ADDR"], os.environ["MASTER_PORT"] = "127.0.0.1", str(port)
     torch.cuda.set_device(rank)
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", rank))
-    from helpers import make_strategy
+    from helpers import load_gold, make_strategy
     from active_learning_b200.engine import Engine
     from active_learning_b200.sharding import ShardGroup
-    gold = dict(np.load(gold_path))
+    gold = load_gold(gold_path)
     n, ev, lab = int(gold["e2e_n"]), gold["e2e_eval_idxs"], gold["e2e_labeled"]
     eng = Engine(rank).comm_init()
     group = ShardGroup()
